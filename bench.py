@@ -2,7 +2,7 @@
 """bench.py -- throughput of the Friture spectral hot path on B200 (one JSON line on stdout).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload combined|stft|bank|gcc]
-                    [--impl ours|reference]
+                    [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of synthetic 48 kHz float32 audio.  The default
 workload is the one BASELINE.json's metric is quoted on ("2048-pt STFT + 30-band 1/3-octave"),
@@ -515,6 +515,15 @@ class Combined:
         self.an.bank.reset()
         return res
 
+    def outputs(self):
+        """What a caller of the step receives: log-power columns (gathered over the ranks at N > 1)
+        and band-level vectors in dB."""
+        if self.gather:
+            if self.transport == "peer":
+                self.an.peer_gather.wait_all()
+            return {"spectrogram_logpower_gathered": self.gathered, "bands_db": self.bands}
+        return {"spectrogram_logpower": self.spec, "bands_db": self.bands}
+
     def roofline(self, peak, peak_src):
         ms = [a.elapsed_time(b) for a, b in self.bank_events]
         if not ms:
@@ -603,6 +612,9 @@ class StftOnly:
         return {"logpower_rel": rel, "ok": rel < 1e-5,
                 "criterion": "max|got-ref| / max(max|ref|, 1) < 1e-5 on %d ch x %d frames" % (cs, fs)}
 
+    def outputs(self):
+        return {"spectrogram_logpower": self.out}
+
     def roofline(self, peak, peak_src):
         if not self.events:
             return None
@@ -680,6 +692,9 @@ class BankOnly:
         return {"band_db_rel": rel, "ok": rel < 1e-5,
                 "criterion": "max|got-ref| / max(max|ref|, 1) < 1e-5 on %d ch x %d blocks" % (cs, fs)}
 
+    def outputs(self):
+        return {"bands_db": self.e}
+
     def roofline(self, peak, peak_src):
         if not self.events:
             return None
@@ -733,9 +748,13 @@ class GccOnly:
         ok = bool((idx == 137).all().item())
         xc = fo.generalized_cross_correlation(self.d0[0].cpu().numpy().astype(np.float64),
                                               self.d1[0].cpu().numpy().astype(np.float64))
-        i_ref, _ = fo.delay_peak(xc)
+        i_ref = fo.delay_peak(xc)[0]
         return {"delays_recovered": ok, "argmax_matches_oracle": bool(int(idx[0].item()) == int(i_ref)),
                 "ok": ok and int(idx[0].item()) == int(i_ref), "criterion": "identical arg-max (known delay 137)"}
+
+    def outputs(self):
+        idx, val, _ = self.res
+        return {"delay_index": idx.double(), "peak_value": val}
 
     def roofline(self, peak, peak_src):
         if not self.events:
@@ -749,6 +768,29 @@ class GccOnly:
 
     def e2e(self, steps, barrier):
         return None, None
+
+
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(outputs, out_dir):
+    """Write each output as <out_dir>/<name>.npy (float32 / float64), DUMP_BYTES in all.  An output
+    larger than its share is viewed as rows of its last dimension (of single elements when one such
+    row alone exceeds the share) and keeps a fixed, seeded sample of those rows in ascending order,
+    written as [rows, width]; two builds run with the same arguments write the same rows."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BYTES // len(outputs) - 4096          # room for the .npy headers
+    for name, t in outputs.items():
+        if t.numel() * t.element_size() > share:
+            width = t.shape[-1] if t.shape[-1] * t.element_size() <= share else 1
+            flat = t.reshape(-1, width)
+            keep = share // (width * t.element_size())
+            rows = np.sort(np.random.default_rng(0).choice(flat.shape[0], keep, replace=False))
+            t = flat[torch.from_numpy(rows).to(t.device)]
+        a = t.detach().cpu().numpy()
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 WORKLOADS = {"combined": Combined, "stft": StftOnly, "bank": BankOnly, "gcc": GccOnly}
@@ -903,7 +945,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-others", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's outputs; the reference arm has none")
     dC, dF = DEFAULTS[args.workload]
     args.channels = args.channels or dC
     args.frames = dF if args.frames is None else args.frames
@@ -960,6 +1008,10 @@ def main():
     time.sleep(0.2)
     sampler.stop()
     clocks = sampler.summary(t_wall0, t_wall1)
+    if args.dump_outputs:       # before the e2e and extra runs reuse the buffers
+        outs = wl.outputs()
+        if rank == 0:
+            dump_outputs(outs, args.dump_outputs)
     t = torch.tensor([total_ms], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

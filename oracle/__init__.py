@@ -7,9 +7,8 @@ product path (``friture_b200`` fails loudly when its CUDA library is missing and
 no CPU fallback).
 
 Parity status: PINNED.  The restatement in :mod:`oracle.friture_oracle` is validated
-against the unmodified reference imported from ``/root/reference`` (see
-``oracle/ref_import.py`` and ``tests/test_oracle_vs_reference.py``, which run in the
-build container) and against golden vectors generated from that reference by
-``oracle/make_golden.py`` and committed under ``tests/golden/`` (these travel to the
-GPU box, where ``/root/reference`` does not exist).
+against golden vectors that ``oracle/make_golden.py`` generates from the unmodified
+reference (imported in place by ``oracle/ref_import.py``) and that are committed under
+``tests/golden/``; ``tests/test_oracle_vs_reference.py`` and ``tests/test_oracle_golden.py``
+check them without the reference tree.
 """

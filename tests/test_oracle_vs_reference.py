@@ -1,17 +1,36 @@
-"""CPU, build container only: the oracle restatement against the UNMODIFIED reference imported in
-place from /root/reference (skipped where the reference tree does not exist, e.g. the GPU box)."""
+"""CPU: the oracle restatement against the UNMODIFIED reference, through what oracle/make_golden.py
+recorded of the reference's outputs (tests/golden/reference_checks.npz): digests where the oracle
+must be bit-identical to the reference (see oracle/digest.py), values where it may differ by
+rounding.  The seeded inputs are regenerated here; their digests are stored with the outputs."""
+import os
+
 import numpy as np
 import pytest
 
 from oracle import friture_oracle as fo
-from oracle import ref_import
+from oracle.digest import digest
 
-pytestmark = pytest.mark.skipif(not ref_import.available(), reason="reference tree not present")
+GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
 @pytest.fixture(scope="module")
 def ref():
-    return ref_import.load()
+    with np.load(os.path.join(GOLD, "reference_checks.npz")) as d:
+        return {k: d[k] for k in d.files}
+
+
+def same(g, key, *arrays):
+    return digest(*arrays) == str(g[key])
+
+
+def seeded(g, key, *arrays):
+    """The regenerated inputs are the ones the reference was run on."""
+    assert same(g, key, *arrays), "%s: numpy's seeded stream changed; rerun oracle/make_golden.py" % key
+
+
+def coeffs(bpo):
+    with np.load(os.path.join(GOLD, "coefficients.npz")) as c:
+        return c["bdec"], c["adec"], list(c["b%d" % bpo]), list(c["a%d" % bpo])
 
 
 def test_analyzelive_all_sizes(ref):
@@ -19,113 +38,113 @@ def test_analyzelive_all_sizes(ref):
         n = 32 * 2 ** k                                   # spectrum_settings.py:61-70
         rng = np.random.default_rng(n)
         x = rng.standard_normal(n)
-        proc = ref.audioproc.audioproc()
-        proc.set_fftsize(n)
-        assert np.array_equal(proc.analyzelive(x.copy()), fo.analyzelive(x))
-        assert np.array_equal(proc.window, fo.hann_window(n))
+        seeded(ref, "analyzelive_x_%d" % n, x)
+        assert same(ref, "analyzelive_%d" % n, fo.analyzelive(x)), n
+        assert same(ref, "window_%d" % n, fo.hann_window(n)), n
 
 
 def test_lfilter_bit_identical(ref):
     from oracle import iir_c
-    P = ref.generated_filters.PARAMS
+    bdec, adec, boct, aoct = coeffs(3)
     rng = np.random.default_rng(0)
     x = rng.standard_normal(700)
-    for b, a in [(P["dec"][0], P["dec"][1]), (P["3"][0][1], P["3"][1][1])]:
-        b, a = np.array(b), np.array(a)
+    seeded(ref, "lfilter_x", x)
+    for name, b, a in [("dec", bdec, adec), ("band", boct[1], aoct[1])]:
         zi = rng.standard_normal(len(b) - 1) * 0.01
-        y0, z0 = ref.lfilter.lfilter_float64_1D(b, a, x, zi.copy())
+        seeded(ref, "lfilter_%s_zi" % name, zi)
         for fn in (fo.lfilter_df2t, fo.lfilter_df2t_loop, iir_c.lfilter):
             y, z = fn(b, a, x, zi.copy())
-            assert np.array_equal(y, y0) and np.array_equal(z, z0), fn
+            assert same(ref, "lfilter_%s" % name, y, z), fn
 
 
 def test_bank_and_smoothing(ref):
-    from friture.filter import octave_filter_bank_decimation, octave_filter_bank_decimation_filtic
-    P = ref.generated_filters.PARAMS
-    bdec, adec = np.array(P["dec"][0]), np.array(P["dec"][1])
     for bpo in (1, 3, 24):
-        boct = [np.array(v) for v in P[str(bpo)][0]]
-        aoct = [np.array(v) for v in P[str(bpo)][1]]
+        bdec, adec, boct, aoct = coeffs(bpo)
         rng = np.random.default_rng(bpo)
-        zr = octave_filter_bank_decimation_filtic(bdec, adec, boct, aoct)
         zo = fo.bank_filtic(bdec, adec, boct, aoct)
-        for _ in range(3):
+        for step in range(3):
             x = rng.standard_normal(512)
-            yr, dr, zr = octave_filter_bank_decimation(bdec, adec, boct, aoct, x, zr)
+            seeded(ref, "bank_bpo%d_x%d" % (bpo, step), x)
             yo, do, zo = fo.octave_filter_bank_decimation(bdec, adec, boct, aoct, x, zo)
-            assert dr == do
-            assert all(np.array_equal(a, b) for a, b in zip(yr, yo))
-            assert all(np.array_equal(a, b) for a, b in zip(zr, zo))
+            assert np.array_equal(do, ref["bank_bpo%d_dec%d" % (bpo, step)])
+            assert same(ref, "bank_bpo%d_y%d" % (bpo, step), yo), (bpo, step)
+            assert same(ref, "bank_bpo%d_z%d" % (bpo, step), zo), (bpo, step)
     k = fo.smoothing_kernel(0.01, 64)
     d = np.random.default_rng(1).random(40)
-    assert ref.exp_smoothing.exp_smoothed_value(k, 0.01, d, 0.3) == fo.exp_smoothed_value(k, 0.01, d, 0.3)
+    seeded(ref, "smoothing_data", d)
+    assert ref["smoothing_value"] == fo.exp_smoothed_value(k, 0.01, d, 0.3)
 
 
 def test_octave_filters_attributes_and_gcc(ref):
-    of = ref.octavefilters.Octave_Filters(3)
     fi, fl, fh = fo.octave_frequencies(27, 3)
-    assert np.array_equal(of.fi, fi) and np.array_equal(of.flow, fl) and np.array_equal(of.fhigh, fh)
-    assert of.get_decs() == fo.get_decs(3)
+    assert same(ref, "of3_fi", fi) and same(ref, "of3_flow", fl) and same(ref, "of3_fhigh", fh)
+    assert fo.get_decs(3) == list(ref["of3_decs"])
     A, B, C = fo.weighting_tables(fi, eps=0.0)
-    assert np.array_equal(of.A, A) and np.array_equal(of.B, B) and np.array_equal(of.C, C)
+    assert same(ref, "of3_A", A) and same(ref, "of3_B", B) and same(ref, "of3_C", C)
     rng = np.random.default_rng(3)
     d0, d1 = rng.standard_normal(24000), rng.standard_normal(24000)
-    xr = ref.correlation.generalized_cross_correlation(d0.copy(), d1.copy())
-    assert np.array_equal(xr, fo.generalized_cross_correlation(d0, d1))
+    seeded(ref, "gcc_x", d0, d1)
+    assert same(ref, "gcc", fo.generalized_cross_correlation(d0, d1))
 
 
-def test_filter_data_matches_reference(ref):
-    """friture_b200/data/filters.npz carries exactly the reference's coefficients."""
+def test_filter_data_matches_reference():
+    """friture_b200/data/filters.npz carries exactly the reference's coefficients
+    (tests/golden/coefficients.npz holds them as the reference's generated_filters.PARAMS)."""
     from friture_b200 import filter_data
-    P = ref.generated_filters.PARAMS
+    bdec_r, adec_r, _, _ = coeffs(3)
     bdec, adec, sos = filter_data.decimator()
-    assert np.array_equal(bdec, np.array(P["dec"][0])) and np.array_equal(adec, np.array(P["dec"][1]))
+    assert np.array_equal(bdec, bdec_r) and np.array_equal(adec, adec_r)
     for bpo in (1, 3, 6, 12, 24):
+        _, _, b_r, a_r = coeffs(bpo)
         b, a, s = filter_data.bands(bpo)
-        assert np.array_equal(b, np.array(P[str(bpo)][0])) and np.array_equal(a, np.array(P[str(bpo)][1]))
+        assert np.array_equal(b, np.array(b_r)) and np.array_equal(a, np.array(a_r))
 
 
 def test_shim_labels_and_attributes_match_reference(ref):
     """Octave_Filters host-side attributes (no GPU needed)."""
     from friture_b200.octavefilters import Octave_Filters
     for bpo in (1, 3, 6, 12, 24):
-        r = ref.octavefilters.Octave_Filters(bpo)
         m = Octave_Filters(bpo)
-        assert m.f_nominal == r.f_nominal
-        for name in ("fi", "flow", "fhigh", "A", "B", "C", "bdec", "adec"):
-            assert np.array_equal(getattr(m, name), getattr(r, name)), name
-        assert all(np.array_equal(x, y) for x, y in zip(m.boct, r.boct))
-        assert all(np.array_equal(x, y) for x, y in zip(m.aoct, r.aoct))
-        assert m.get_decs() == r.get_decs() and m.nbands == r.nbands
+        assert m.f_nominal == list(ref["of%d_f_nominal" % bpo])
+        for name in ("fi", "flow", "fhigh", "A", "B", "C", "bdec", "adec", "boct", "aoct"):
+            assert same(ref, "of%d_%s" % (bpo, name), getattr(m, name)), (bpo, name)
+        assert m.get_decs() == list(ref["of%d_decs" % bpo]) and m.nbands == int(ref["of%d_nbands" % bpo])
     from friture_b200 import audioproc
-    pr, pm = ref.audioproc.audioproc(), audioproc()
+    pm = audioproc()
     for n in (1024, 2048):
-        pr.set_fftsize(n)
         pm.set_fftsize(n)
         for name in ("window", "freq", "A", "B", "C", "size_sq", "fft_size"):
-            assert np.array_equal(getattr(pm, name), getattr(pr, name)), name
+            assert same(ref, "audioproc%d_%s" % (n, name), getattr(pm, name)), (n, name)
 
 
 def test_live_fft_bank_restatement_and_fir_data(ref):
     """oracle.octave_filter_bank_decimation_fft == the unmodified reference's Octave_Filters.filter
     (live FFT overlap-add path, friture/filter.py:136-247) to 1e-15; the direct FIR form the GPU
-    kernel computes equals it to rounding; data/fir.npz holds the reference's taps."""
+    kernel computes equals it to rounding; data/fir.npz holds the reference's taps.  The reference's
+    band outputs are stored whole at 1 and 3 bands per octave, as 16 fixed positions of every band
+    at 24, with every band's L2 norm and peak; the per-element bounds imply the norm bounds
+    (triangle inequality) and bound the direct form against the restatement everywhere."""
     from friture_b200 import filter_data
-    from oracle import friture_oracle as fo
     assert fo.fft_bank_sizes() == [1536, 1024, 768, 640, 576, 576, 540, 540, 540]
     rng = np.random.default_rng(1)
     for bpo in (1, 3, 24):
         boct_fir, bdec_fir = filter_data.fir_taps(bpo)
-        of = ref.octavefilters.Octave_Filters(bpo)
-        assert np.array_equal(np.stack(of._boct_fir), boct_fir) and np.array_equal(of._bdec_fir, bdec_fir)
+        assert same(ref, "fft%d_taps" % bpo, boct_fir, bdec_fir)
         oo, od = fo.fft_bank_state(bpo)
         hist = [np.zeros(511) for _ in range(9)]
         for blk in range(5):
             x = rng.standard_normal(512 if blk % 2 else 1024) * 0.1
-            yr, decr = of.filter(x)
+            seeded(ref, "fft%d_x%d" % (bpo, blk), x)
             y, dec, oo, od = fo.octave_filter_bank_decimation_fft(boct_fir, bdec_fir, x, oo, od)
             y2, hist = fo.fir_bank_direct(boct_fir, bdec_fir, x, hist)
-            assert dec == decr
-            for a, b, c in zip(y, yr, y2):
-                assert np.max(np.abs(a - b)) < 1e-14
-                assert np.max(np.abs(c - b)) < 1e-12 * max(np.max(np.abs(b)), 1.0)
+            assert np.array_equal(dec, ref["fft%d_dec%d" % (bpo, blk)])
+            val = ref["fft%d_val%d" % (bpo, blk)]
+            sel = ref.get("fft%d_idx%d" % (bpo, blk), slice(None))
+            lens, norm, peak = (ref["fft%d_%s%d" % (bpo, k, blk)] for k in ("len", "norm", "peak"))
+            assert [len(v) for v in y] == list(lens) == [len(v) for v in y2]
+            tol2 = np.repeat(1e-12 * np.maximum(peak, 1.0), lens)
+            yc, y2c = np.concatenate(y), np.concatenate(y2)
+            assert np.max(np.abs(yc[sel] - val)) < 1e-14
+            assert np.all(np.abs(y2c[sel] - val) < tol2[sel])
+            assert np.all(np.abs(y2c - yc) < tol2 + 1e-14)
+            assert np.all(np.abs([np.linalg.norm(v) for v in y] - norm) <= 1e-14 * np.sqrt(lens))
