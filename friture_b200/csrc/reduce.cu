@@ -59,13 +59,15 @@ spectrum_reduce_kernel(const float *__restrict__ power, long long stride_c, long
     const int c = blockIdx.x;
     const float *p = power + (size_t)c * stride_c;
     float *d = disp + (size_t)c * nbins;
-    const float om = 1.0f - alpha;
     float best = -INFINITY;
     int besti = 0x7fffffff;
     for (int k = threadIdx.x; k < nbins; k += blockDim.x) {
         float s = d[k];
-        for (int f = 0; f < n_frames; f++)   // s <- alpha x + (1-alpha) s  (exp_smoothing.py:59-107)
-            s = fmaf(alpha, __ldg(p + (size_t)f * stride_f + k), om * s);
+        // s <- alpha x + (1-alpha) s  (exp_smoothing.py:59-107), in complement form s + alpha (x - s):
+        // a float32-rounded 1-alpha would shift the time constant by up to 1e-3 at alpha ~ 3.5e-5
+        // (N = 32, 5 s) and bias the steady state (tests/test_spectrum_host.py)
+        for (int f = 0; f < n_frames; f++)
+            s = fmaf(alpha, __ldg(p + (size_t)f * stride_f + k) - s, s);
         d[k] = s;
         s_sp[k] = s;
         float v = 3.01029995663981195f * lg2_fast(s + 1e-30f);   // spectrum.py:95-101
